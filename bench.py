@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (restated)
+    python bench.py ... --dump-outputs DIR                   # also writes the last timed step's match list (.npy)
 
 A "step" is one blocking Matcher::match_list_parallel call (frz_match_list_parallel_rank; at N = 1 this is
 Matcher::match_list) over one synthetic haystack list of BASELINE.json configs[2] shape per GPU — needle 'deadbeef',
@@ -68,7 +69,13 @@ def parse_args():
     ap.add_argument("--shards-per-gpu", type=int, default=1,
                     help="each GPU holds this many consecutive logical shards of --n haystacks (seeds consecutive): "
                          "`--gpus 1 --shards-per-gpu 8` matches the very list `--gpus 8` shards over 8 GPUs (strong scaling)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the ordered match list of the last timed step to DIR as .npy files "
+                         "(see dump_outputs), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 class ClockSampler:
@@ -223,6 +230,27 @@ def calibration(cb, cfg):
                     "(BENCHMARKS.md:124)"}
 
 
+DUMP_BYTES = 64_000_000   # --dump-outputs: all files together stay below this
+
+
+def dump_outputs(out_dir, matches):
+    """Writes an ordered match list (MATCH_DTYPE) as DIR/matches_{index,score,exact}.npy (index float64, score and exact
+    float32, all exact) and DIR/matches_count.npy (the list's length).  A list too long for DUMP_BYTES is replaced by a
+    fixed, seeded sample of its rows, and DIR/matches_position.npy holds where the sampled rows sit in the full list."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(matches)
+    max_rows = (DUMP_BYTES - 4096) // (8 + 4 + 4 + 8)   # index, score, exact, position; 4 KB for the .npy headers
+    fields = {"count": np.array([n], dtype=np.float64)}
+    if n > max_rows:
+        pos = np.sort(np.random.default_rng(12345).choice(n, max_rows, replace=False))
+        matches = matches[pos]
+        fields["position"] = pos.astype(np.float64)
+    fields.update(index=matches["index"].astype(np.float64), score=matches["score"].astype(np.float32),
+                  exact=matches["exact"].astype(np.float32))
+    for name, arr in fields.items():
+        np.save(os.path.join(out_dir, f"matches_{name}.npy"), arr)
+
+
 def run_reference(args):
     """The reference's own CPU implementation of the path (restated; no Rust toolchain here), all host threads,
     on a bounded sample of the same workload."""
@@ -262,6 +290,8 @@ def run_reference(args):
                                        f"the process's CPUs round-robin), emulating the {lanes}-lane reference backend",
                              "calibration": calibration(cb, cfg)},
             "e2e": {"value": value, "unit": "haystacks/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     print(json.dumps(line))
 
 
@@ -412,8 +442,9 @@ def run_ours(args):
     est = (time.perf_counter() - t0) / 5
     n_roll = bcast_int(min(4000, max(5, int(0.4 / max(est, 1e-5)))))
 
-    def timed(fn, steps, clocks=False):
-        """pre-roll, K timed steps between CUDA events, post-roll — all fixed counts; max over ranks."""
+    def timed(fn, steps, clocks=False, last=None):
+        """pre-roll, K timed steps between CUDA events, post-roll — all fixed counts; max over ranks.  `last` receives the
+        last timed step's result before the post-roll runs."""
         sampler = ClockSampler(local) if clocks and rank == 0 else None
         barrier()
         if sampler:
@@ -434,6 +465,8 @@ def run_ours(args):
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
+        if last is not None:
+            last(r)
         if clocks:
             for _ in range(n_roll):
                 fn()
@@ -441,7 +474,13 @@ def run_ours(args):
         c = sampler.stop() if sampler else None
         return max_over_ranks(ms), r, c
 
-    ms, n_matches, clocks = timed(step, args.steps, clocks=True)
+    last_list = {}
+
+    def keep_last(count):   # --dump-outputs: the merged list the last timed step landed in the shared host buffer
+        if args.dump_outputs and rank == 0:
+            last_list["matches"] = np.array(out_h[:count])
+
+    ms, n_matches, clocks = timed(step, args.steps, clocks=True, last=keep_last)
     if clocks is not None:
         clocks["window"] = f"{n_roll} identical pre-roll steps + timed region + {n_roll} identical post-roll steps"
     value = n * world * args.steps / (ms / 1e3)
@@ -545,6 +584,8 @@ def run_ours(args):
                                  "AND the match pipeline (tile ranges are matched as they land; only the sort waits for the last chunk)"},
                 "gpu_launches": int(round(launches_per_step * args.steps)),
                 "roofline": roofline, "cpu_baseline": cpu, "parity": parity}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last_list["matches"])
         print(json.dumps(line), flush=True)
     barrier()
     comm.host_free(out_h)
