@@ -62,10 +62,9 @@ static int parallel_demo(int n_gpus) {
         fprintf(stderr, "parallel demo: %s: %s\n", frz_status_str(st), frz_last_error());
     } else {
         const int same = n_seq == n_par && memcmp(seq, par, (size_t)n_seq * sizeof *seq) == 0;
-        static const char* const forms[] = {"ncclAllGather + merge", "NCCL slice exchange", "P2P placement over NVLink", "direct placement into the mapped host buffer"};
         const int mode = frz_comm_exchange_mode(comm);
         printf("match_list_parallel over %d GPU(s): %llu matches, parallel == sequential: %s (exchange: %s)\n", n_gpus, (unsigned long long)n_par,
-               same ? "yes" : "NO", n_gpus > 1 && mode >= 0 && mode <= 3 ? forms[mode] : "n/a");
+               same ? "yes" : "NO", n_gpus == 1 ? "n/a" : mode == 2 ? "P2P placement over NVLink" : "ncclAllGather + merge");
         rc = same ? 0 : 4;
     }
     for (int g = 0; g < 64; g++) frz_corpus_destroy(shards[g]);

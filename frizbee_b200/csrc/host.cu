@@ -1420,10 +1420,8 @@ frz_status streamed_after_chunk(void* ctx, uint32_t t0, uint32_t t1, bool last) 
 
 namespace {
 bool streamed_eligible(const frz_matcher* m, uint64_t n, uint32_t index_offset) {
-    static int knob = -1;   // FRZ_E2E_STREAM=0: ingest first, then match (the A/B partner)
-    if (knob < 0) { const char* e = getenv("FRZ_E2E_STREAM"); knob = e ? atoi(e) : 1; }
     const uint8_t sort = m->config.sort;
-    return knob != 0 && m->compiled.size() == 1 && !m->compiled[0].negated && !m->compiled[0].unicode &&
+    return m->compiled.size() == 1 && !m->compiled[0].negated && !m->compiled[0].unicode &&
            (sort == FRZ_SORT_INDEX_ASC || sort == FRZ_SORT_SCORE_THEN_INDEX_ASC) &&   // reversed lists need the final total per element
            n >= 64 * FRZ_TILE && (uint64_t)n + index_offset <= 0xFFFFFFFFull;
 }

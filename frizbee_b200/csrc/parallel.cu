@@ -13,12 +13,10 @@
 //
 // Host-out calls (the caller wants the list in host memory, the bench's `value`) do better than gather-then-merge:
 // every rank's per-score table crosses the shared host block, after which every rank KNOWS the merged position of each
-// of its matches, and ONE kernel (k_place) stores them straight to where they belong — into the caller's pinned + mapped
-// HOST buffer itself (direct form: zero-copy stores over each GPU's own PCIe link, no peer traffic and no separate
-// device→host copy at all), or, when the buffer is not mapped, into the peer GPUs' slice buffers over NVLink (P2P stores
-// into cudaIpc-mapped / peer-enabled memory, then every GPU copies its slice out) — the k-way merge and the exchange are
-// the same pass, no NCCL kernel, no receive buffer, no second scatter.  The all-gather form remains for device-out calls
-// and as the fallback (FRZ_PARALLEL_EXCHANGE=direct|p2p|slices|allgather).
+// of its matches, and ONE kernel (k_place) stores them straight into the peer GPUs' slice buffers over NVLink (P2P stores
+// into cudaIpc-mapped / peer-enabled memory), after which every GPU copies its slice out — the k-way merge and the exchange
+// are the same pass, no NCCL kernel, no receive buffer, no second scatter.  The all-gather form remains for device-out
+// calls and as the fallback when peer memory cannot be mapped (FRZ_PARALLEL_EXCHANGE=allgather forces it).
 //
 // The only per-step collective is that all-gather.  The match counts (the `Vec` lengths the k-merge reads) are
 // published by each GPU into a small pinned host block shared by all ranks — a 1-thread kernel right after the tile
@@ -70,10 +68,6 @@ struct NcclApi {
     decltype(&ncclCommInitAll) CommInitAll = nullptr;
     decltype(&ncclCommDestroy) CommDestroy = nullptr;
     decltype(&ncclAllGather) AllGather = nullptr;
-    decltype(&ncclSend) Send = nullptr;
-    decltype(&ncclRecv) Recv = nullptr;
-    decltype(&ncclGroupStart) GroupStart = nullptr;
-    decltype(&ncclGroupEnd) GroupEnd = nullptr;
     decltype(&ncclGetErrorString) GetErrorString = nullptr;
     decltype(&ncclGetVersion) GetVersion = nullptr;
 };
@@ -102,10 +96,6 @@ NcclApi& nccl_api() {
         api.CommInitAll = reinterpret_cast<decltype(api.CommInitAll)>(sym("ncclCommInitAll"));
         api.CommDestroy = reinterpret_cast<decltype(api.CommDestroy)>(sym("ncclCommDestroy"));
         api.AllGather = reinterpret_cast<decltype(api.AllGather)>(sym("ncclAllGather"));
-        api.Send = reinterpret_cast<decltype(api.Send)>(sym("ncclSend"));
-        api.Recv = reinterpret_cast<decltype(api.Recv)>(sym("ncclRecv"));
-        api.GroupStart = reinterpret_cast<decltype(api.GroupStart)>(sym("ncclGroupStart"));
-        api.GroupEnd = reinterpret_cast<decltype(api.GroupEnd)>(sym("ncclGroupEnd"));
         api.GetErrorString = reinterpret_cast<decltype(api.GetErrorString)>(sym("ncclGetErrorString"));
         api.GetVersion = reinterpret_cast<decltype(api.GetVersion)>(sym("ncclGetVersion"));
     });
@@ -164,31 +154,6 @@ __global__ void __launch_bounds__(256) k_publish_table(volatile uint32_t* dst, c
     }
 }
 
-// Slice form of the k-way merge: this rank received, from every run q, exactly the elements [a_q, a_q + n_q) that land in
-// its slice [lo, hi) of the merged list.  Element i of piece q with score s goes to
-//     pos0[q][s] + (a_q + i - gt[q][s]) - lo
-// (pos0 = merged position of the first element of run q's score-s block, gt = how many of run q score higher than s).
-struct SliceMeta {
-    uint32_t off[kMaxWorld];   // start of piece q in the receive buffer
-    uint32_t n[kMaxWorld];     // its length
-    uint32_t a[kMaxWorld];     // its first element's index inside run q
-    unsigned long long lo;
-};
-__global__ void __launch_bounds__(256) k_slice_scatter(const FrzMatchDev* __restrict__ recv, const __grid_constant__ SliceMeta meta,
-                                                       const uint32_t* __restrict__ gt, const unsigned long long* __restrict__ pos0,
-                                                       int bins, FrzMatchDev* __restrict__ out) {
-    const int q = blockIdx.y;
-    const FrzMatchDev* piece = recv + meta.off[q];
-    const uint32_t n = meta.n[q], a = meta.a[q];
-    const uint32_t* gtq = gt + (size_t)q * bins;
-    const unsigned long long* p0q = pos0 + (size_t)q * bins;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const FrzMatchDev m = piece[i];
-        const uint32_t s = bins > 1 ? min((uint32_t)m.score, (uint32_t)bins - 1) : 0u;
-        out[p0q[s] + (a + i - gtq[s]) - meta.lo] = m;
-    }
-}
-
 // ---- P2P placement: the exchange and the k-way merge in one pass over peer memory ------------------------------------
 // Rank q holds run q sorted; with every rank's score table it knows pos0[s] (merged position of the first element of its
 // score-s block) and gt[s] (how many of its elements score higher), so element i with score s belongs at merged position
@@ -209,28 +174,13 @@ struct PlaceMeta {
     unsigned long long total;
     int world, rank, bins, parity;
 };
-// DIRECT form (template, opt-in with FRZ_PARALLEL_EXCHANGE=direct): the destination is the caller's HOST buffer itself (pinned +
-// mapped, zero-copy stores over this GPU's own PCIe link): element i goes to host_out[pos0[s] + (i - gt[s])].  No peer
-// memory, no flags, no separate device→host copy, and no rank waits for another rank's run before its own bytes move.
-// Measured slower than the peer form on B200 (SM-issued posted writes reach ~30 GB/s, the copy engine ~52 GB/s:
-// profiles/r02o_bench_n2_direct.json vs r02o_bench_n2_p2p.json), so it is not the default.
-template <bool DIRECT>
 __global__ void __launch_bounds__(256) k_place(const FrzMatchDev* __restrict__ run, unsigned long long n, const __grid_constant__ PlaceMeta meta,
                                                const unsigned long long* __restrict__ pos0, const uint32_t* __restrict__ gt,
-                                               unsigned long long seq, unsigned long long timeout_ns, volatile unsigned long long* err_slot,
-                                               FrzMatchDev* __restrict__ host_out) {
+                                               unsigned long long seq, unsigned long long timeout_ns, volatile unsigned long long* err_slot) {
     __shared__ unsigned long long lo_s[kMaxWorld + 1];
     __shared__ FrzMatchDev* dst_s[kMaxWorld];
     __shared__ int last_s;
     const int world = meta.world, bins = meta.bins;
-    if constexpr (DIRECT) {
-        for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (unsigned long long)gridDim.x * blockDim.x) {
-            const FrzMatchDev m = run[i];
-            const uint32_t s = bins > 1 ? min((uint32_t)m.score, (uint32_t)bins - 1) : 0u;
-            host_out[pos0[s] + (i - gt[s])] = m;
-        }
-        return;   // kernel completion + the stream-ordered "landed" flag make the stores visible to the host
-    }
     for (int i = threadIdx.x; i <= meta.world; i += blockDim.x) lo_s[i] = meta.lo[i];
     for (int i = threadIdx.x; i < meta.world; i += blockDim.x) dst_s[i] = reinterpret_cast<FrzMatchDev*>(meta.peer[i] + kPlaceHeaderBytes);
     __syncthreads();
@@ -317,21 +267,15 @@ struct RankCtx {
     FrzMatchDev* merged = nullptr;
     uint64_t merged_cap = 0;
     FrzMergeScratch merge;
-    // slice exchange (host-out calls): pieces received from every run, device copies of the gt / pos0 tables, pinned staging
-    FrzMatchDev* recv = nullptr;
-    uint64_t recv_cap = 0;
-    uint32_t* d_gt = nullptr;               // (d_pos0 and d_gt are one allocation, h_pos0 and h_gt one pinned staging block:
-    unsigned long long* d_pos0 = nullptr;   //  the tables travel in ONE host→device copy)
-    uint32_t* h_gt = nullptr;
+    // P2P placement (host-out calls): my run's pos0 and gt tables (pos0[0, bins) then gt[0, bins) in one allocation, staged in
+    // one pinned block: they travel in ONE host→device copy); my slice buffer (header + elements), exported to the peers;
+    // theirs mapped here
+    unsigned long long* d_pos0 = nullptr;
     unsigned long long* h_pos0 = nullptr;
-    // P2P placement (host-out calls): my slice buffer (header + elements), exported to the peers; theirs mapped here
     unsigned char* place_raw = nullptr;
     uint64_t place_cap = 0;                 // elements
     unsigned char* peer_raw[kMaxWorld] = {};
     bool peer_ipc[kMaxWorld] = {};          // opened with cudaIpcOpenMemHandle (multi-process form)
-    const void* direct_for = nullptr;       // host `out` pointer (and capacity) the direct form was last negotiated for
-    uint64_t direct_cap = 0;
-    FrzMatchDev* direct_dev = nullptr;      // its device-side address (nullptr: not mapped on some rank → peer / NCCL forms)
     uint32_t* table_dev = nullptr;          // device-side address of the shared table block
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
     bool ev_valid = false;
@@ -359,11 +303,8 @@ struct frz_comm {
     volatile uint64_t* ctrl_host = nullptr;
     HostBlock tables;             // [parity][rank][kTableBins] uint32: every rank's score table of the current step
     volatile uint32_t* tables_host = nullptr;
-    bool slice_exchange = true;   // FRZ_PARALLEL_EXCHANGE=allgather forces the all-gather form for host-out calls too
     bool p2p_exchange = true;     // host-out calls place matches straight into the peers' slice buffers (k_place); cleared by
-                                  // FRZ_PARALLEL_EXCHANGE=slices|allgather, or when peer access / cudaIpc is unavailable
-    bool direct_exchange = true;  // host-out calls store matches straight into the caller's mapped host buffer (k_place<DIRECT>);
-                                  // needs `out` to be pinned + mapped on every rank (frz_comm_host_alloc memory is)
+                                  // FRZ_PARALLEL_EXCHANGE=allgather, or when peer access / cudaIpc is unavailable
     // local form: rendezvous of the worker threads (allgather_words)
     std::mutex tb_mu;
     std::condition_variable tb_cv;
@@ -401,10 +342,9 @@ void rank_release(RankCtx& r) {
         r.peer_raw[q] = nullptr; r.peer_ipc[q] = false;
     }
     cudaFree(r.place_raw); r.place_raw = nullptr; r.place_cap = 0;
-    cudaFree(r.run); cudaFree(r.d_count); cudaFree(r.gathered); cudaFree(r.merged); cudaFree(r.recv); cudaFree(r.d_pos0);
+    cudaFree(r.run); cudaFree(r.d_count); cudaFree(r.gathered); cudaFree(r.merged); cudaFree(r.d_pos0);
     if (r.h_pos0) cudaFreeHost(r.h_pos0);
-    r.run = nullptr; r.d_count = nullptr; r.gathered = nullptr; r.merged = nullptr; r.recv = nullptr; r.d_gt = nullptr; r.d_pos0 = nullptr;
-    r.h_gt = nullptr; r.h_pos0 = nullptr;
+    r.run = nullptr; r.d_count = nullptr; r.gathered = nullptr; r.merged = nullptr; r.d_pos0 = nullptr; r.h_pos0 = nullptr;
     r.merge.release();
     for (auto& e : r.ev) { if (e) cudaEventDestroy(e); e = nullptr; }
     if (r.side) cudaStreamDestroy(r.side);
@@ -472,38 +412,12 @@ frz_status allgather_words(frz_comm* c, RankCtx& r, const uint64_t* mine, int n_
     return FRZ_OK;
 }
 
-// Direct form: is the caller's `out` buffer addressable from every rank's GPU?  Negotiated once per buffer (collective: the
-// ranks make the same calls with the same shared buffer, so they reach this together); any rank that cannot map it turns
-// the form off for that buffer on all ranks.
-frz_status negotiate_direct(frz_comm* c, RankCtx& r, const frz_match* out_host, uint64_t cap, FrzMatchDev** dev) {
-    *dev = nullptr;
-    if (!c->direct_exchange || !out_host) return FRZ_OK;
-    if (r.direct_for == out_host && r.direct_cap == cap) { *dev = r.direct_dev; return FRZ_OK; }
-    void* dp = nullptr;
-    uint64_t ok = cudaHostGetDevicePointer(&dp, const_cast<frz_match*>(out_host), 0) == cudaSuccess && dp ? 1 : 0;
-    if (ok && cap) {   // the whole buffer, not just its first page
-        void* dp2 = nullptr;
-        ok = cudaHostGetDevicePointer(&dp2, const_cast<frz_match*>(out_host + (cap - 1)), 0) == cudaSuccess &&
-             dp2 == static_cast<void*>(static_cast<FrzMatchDev*>(dp) + (cap - 1)) ? 1 : 0;
-    }
-    if (!ok) cudaGetLastError();
-    uint64_t all[kMaxWorld];
-    FRZ_TRY(allgather_words(c, r, &ok, 1, all));
-    for (int q = 0; q < c->world; q++) ok = ok && all[q] == 1;
-    r.direct_for = out_host;
-    r.direct_cap = cap;
-    r.direct_dev = ok ? static_cast<FrzMatchDev*>(dp) : nullptr;
-    *dev = r.direct_dev;
-    return FRZ_OK;
-}
-
 // Slice buffers of the P2P placement: every rank owns `header + cap elements`, every other rank maps it (local form: peer
 // access between the devices of one process; multi-process form: cudaIpc handles exchanged over the communicator).
 // Grow-only and COLLECTIVE: `need` is derived from the step's total match count, which every rank knows, so all ranks
-// take the same branch.  On any failure every rank clears c->p2p_exchange and the caller falls back to the NCCL forms.
+// take the same branch.  On any failure every rank clears c->p2p_exchange and the caller falls back to the all-gather.
 frz_status ensure_place_buffers(frz_comm* c, RankCtx& r, uint64_t need, bool* ready) {
     *ready = false;
-    if (!c->p2p_exchange) return FRZ_OK;
     if (r.place_cap >= need) { *ready = true; return FRZ_OK; }
     const int world = c->world;
     FRZ_CUDA_TRY(cudaDeviceSynchronize());   // nothing of mine may still read or write the old buffers
@@ -564,7 +478,7 @@ frz_status ensure_place_buffers(frz_comm* c, RankCtx& r, uint64_t need, bool* re
 // one memory node that node's DRAM write bandwidth and the socket interconnect are the limit (measured at 8 GPUs: the
 // eight concurrent 6 MB slice copies took 0.28 ms instead of 0.11 ms, profiles/r02g_bench_n8.json; 0.21 ms with the
 // first-touch placement below, whose parts only line up with the slices when the list fills the buffer,
-// profiles/r02l_bench_n8.json).  See numa_policy().
+// profiles/r02l_bench_n8.json).  See first_touch_near().
 int gpu_numa_node(int device) {
     char bus[32] = {0};
     if (cudaDeviceGetPCIBusId(bus, sizeof bus, device) != cudaSuccess) { cudaGetLastError(); return -1; }
@@ -596,50 +510,12 @@ bool node_cpus(int node, cpu_set_t* set) {   // parses /sys/devices/system/node/
     fclose(f);
     return n > 0;
 }
-// Page placement policy of the shared host buffers (FRZ_HOST_NUMA):
-//   touch (default)  rank r first-touches the r-th part of the buffer from a CPU of its GPU's node (exact only when the list
-//                    fills the buffer: slices are fractions of the USED part)
-//   interleave       pages alternate over the memory nodes (mbind MPOL_INTERLEAVE before the first touch): every GPU's slice
-//                    is half local, half remote, wherever the slice boundaries of a step fall
-//   none             wherever the kernel puts them
-// Measured at 8 GPUs (profiles/r02n_*, FRZ_PARALLEL_DEBUG=1 prints where the pages are): rank 0's 6 MB slice copy takes
-// 0.19 ms with touch or none (the ranks happened to run on their GPU's node) and 0.26 ms interleaved, against 0.115 ms alone —
-// and the step is 0.711-0.717 ms with all three: page placement is not what slows eight concurrent slice copies down.
-enum { kNumaInterleave = 0, kNumaTouch = 1, kNumaNone = 2 };
-int numa_policy() {
-    static int p = -1;
-    if (p < 0) {
-        const char* e = getenv("FRZ_HOST_NUMA");
-        p = !e ? kNumaTouch : strcmp(e, "interleave") == 0 ? kNumaInterleave : strcmp(e, "none") == 0 ? kNumaNone : kNumaTouch;
-    }
-    return p;
-}
+// Page placement of the shared host buffers: rank r first-touches the r-th part of the buffer from a CPU of its GPU's node
+// (exact only when the list fills the buffer: slices are fractions of the USED part).  Measured at 8 GPUs (profiles/r02n_*,
+// FRZ_PARALLEL_DEBUG=1 prints where the pages are): rank 0's 6 MB slice copy takes 0.19 ms with this placement against
+// 0.26 ms with the pages interleaved over the memory nodes and 0.115 ms alone.  Leaving placement to the kernel tied only
+// because the ranks happened to run on their GPU's node; in the one-process form it puts every page on one node.
 bool numa_debug() { static int d = -1; if (d < 0) { const char* e = getenv("FRZ_PARALLEL_DEBUG"); d = e && atoi(e) ? 1 : 0; } return d == 1; }
-// nodes that have memory: /sys/devices/system/node/has_memory ("0-1"); 0 when unknown
-unsigned long memory_node_mask() {
-    FILE* f = fopen("/sys/devices/system/node/has_memory", "r");
-    if (!f) f = fopen("/sys/devices/system/node/online", "r");
-    if (!f) return 0;
-    unsigned long mask = 0;
-    int a = 0, b = 0;
-    for (;;) {
-        if (fscanf(f, "%d", &a) != 1) break;
-        b = a;
-        int ch = fgetc(f);
-        if (ch == '-') { if (fscanf(f, "%d", &b) != 1) break; ch = fgetc(f); }
-        for (int n = a; n <= b && n < (int)(8 * sizeof mask); n++) mask |= 1ul << n;
-        if (ch != ',') break;
-    }
-    fclose(f);
-    return mask;
-}
-// mbind(MPOL_INTERLEAVE) over the memory nodes; raw syscall (no libnuma in the image).  false = unavailable (one node, no permission)
-bool interleave_pages(void* ptr, uint64_t bytes) {
-    const unsigned long mask = memory_node_mask();
-    if (__builtin_popcountl(mask) < 2) return false;
-    constexpr int kMpolInterleave = 3;
-    return syscall(SYS_mbind, ptr, (unsigned long)bytes, kMpolInterleave, &mask, (unsigned long)(8 * sizeof mask + 1), 0u) == 0;
-}
 // node of the page holding `addr` (move_pages with a null target = query), -1 when unknown
 int page_node(void* addr) {
     void* page = reinterpret_cast<void*>(reinterpret_cast<uintptr_t>(addr) & ~4095ull);
@@ -648,12 +524,12 @@ int page_node(void* addr) {
     return status;
 }
 // touches [lo, hi) of `ptr` (one byte per page, value preserved as zero) from a CPU near `device`, then restores the affinity
-void first_touch_near(int device, unsigned char* ptr, uint64_t lo, uint64_t hi, bool pin_near) {
+void first_touch_near(int device, unsigned char* ptr, uint64_t lo, uint64_t hi) {
     cpu_set_t old_set, near_set;
     const bool have_old = sched_getaffinity(0, sizeof old_set, &old_set) == 0;
     const int node = gpu_numa_node(device);
     bool moved = false;
-    if (pin_near && have_old && node >= 0 && node_cpus(node, &near_set)) {
+    if (have_old && node >= 0 && node_cpus(node, &near_set)) {
         cpu_set_t both;
         CPU_AND(&both, &near_set, &old_set);   // stay inside whatever the launcher allowed
         if (CPU_COUNT(&both) > 0) moved = sched_setaffinity(0, sizeof both, &both) == 0;
@@ -661,8 +537,8 @@ void first_touch_near(int device, unsigned char* ptr, uint64_t lo, uint64_t hi, 
     for (uint64_t off = lo & ~4095ull; off < hi; off += 4096) ptr[off] = 0;
     if (moved) sched_setaffinity(0, sizeof old_set, &old_set);
     if (numa_debug() && hi > lo)
-        fprintf(stderr, "[frz numa] device %d: sysfs node %d, affinity %s, policy %d; pages of [%llu, %llu): first on node %d, middle %d, last %d\n",
-                device, node, moved ? "moved" : "unchanged", numa_policy(), (unsigned long long)lo, (unsigned long long)hi,
+        fprintf(stderr, "[frz numa] device %d: sysfs node %d, affinity %s; pages of [%llu, %llu): first on node %d, middle %d, last %d\n",
+                device, node, moved ? "moved" : "unchanged", (unsigned long long)lo, (unsigned long long)hi,
                 page_node(ptr + lo), page_node(ptr + (lo + hi) / 2), page_node(ptr + hi - 1));
 }
 
@@ -676,10 +552,8 @@ frz_status host_block_alloc(frz_comm* c, uint64_t bytes, HostBlock* out) {
         b.ptr = mmap(nullptr, bytes, PROT_READ | PROT_WRITE, MAP_PRIVATE | MAP_ANONYMOUS, -1, 0);
         if (b.ptr == MAP_FAILED) return frz_fail(FRZ_ERR_OOM, "cannot map %llu bytes of host memory", (unsigned long long)bytes);
         const int world = c->world;
-        const bool inter = numa_policy() == kNumaInterleave && interleave_pages(b.ptr, bytes);
         for (int g = 0; g < world; g++)
-            first_touch_near(c->ranks[g].device, static_cast<unsigned char*>(b.ptr), bytes * (uint64_t)g / world, bytes * (uint64_t)(g + 1) / world,
-                             !inter && numa_policy() == kNumaTouch);
+            first_touch_near(c->ranks[g].device, static_cast<unsigned char*>(b.ptr), bytes * (uint64_t)g / world, bytes * (uint64_t)(g + 1) / world);
         FRZ_TRY(set_device(c->ranks[0].device));
         if (cudaHostRegister(b.ptr, bytes, cudaHostRegisterPortable | cudaHostRegisterMapped) != cudaSuccess) {
             cudaGetLastError();
@@ -710,13 +584,10 @@ frz_status host_block_alloc(frz_comm* c, uint64_t bytes, HostBlock* out) {
         b.ptr = mmap(nullptr, bytes, PROT_READ | PROT_WRITE, MAP_SHARED, b.fd, 0);
         if (b.ptr == MAP_FAILED) { b.ptr = nullptr; ok = 0; }
     }
-    // page placement (numa_policy above): the policy is set on every rank's mapping, every rank touches ITS part of the
-    // segment (shared-memory pages follow the policy of the mapping that faults them in), everybody waits, then everybody pins
-    if (ok) {
-        const bool inter = numa_policy() == kNumaInterleave && interleave_pages(b.ptr, bytes);
+    // page placement (first_touch_near above): every rank touches ITS part of the segment, everybody waits, then everybody pins
+    if (ok)
         first_touch_near(c->ranks[0].device, static_cast<unsigned char*>(b.ptr), bytes * (uint64_t)c->rank / c->world,
-                         bytes * (uint64_t)(c->rank + 1) / c->world, !inter && numa_policy() == kNumaTouch);
-    }
+                         bytes * (uint64_t)(c->rank + 1) / c->world);
     std::vector<uint64_t> oks(c->world);
     FRZ_TRY(exchange_words(c, &ok, 1, oks.data()));
     if (ok) {
@@ -742,13 +613,9 @@ frz_status comm_finish_setup(frz_comm* c) {
     { const char* e = getenv("FRZ_PARALLEL_FORCE_NCCL"); c->force_nccl = e && atoi(e) != 0; }
     FRZ_TRY(host_block_alloc(c, kCtrlBytes, &c->ctrl));
     c->ctrl_host = reinterpret_cast<volatile uint64_t*>(c->ctrl.ptr);
-    {   // host-out exchange: p2p (default) → slices (NCCL send/recv) → allgather
+    {   // host-out exchange: p2p (default) → allgather
         const char* e = getenv("FRZ_PARALLEL_EXCHANGE");
-        c->slice_exchange = !(e && strcmp(e, "allgather") == 0);
-        c->p2p_exchange = c->slice_exchange && !(e && strcmp(e, "slices") == 0) && c->world > 1;
-        // direct form: opt-in.  Measured on 2 B200s (profiles/r02o_*): the SMs' zero-copy stores move the 6 MB of a rank at
-        // ~30 GB/s against ~52 GB/s for the copy engine, 0.211 ms against 0.045 (k_place) + 0.115 (slice copy) for the P2P form
-        c->direct_exchange = c->slice_exchange && c->world > 1 && e && strcmp(e, "direct") == 0;
+        c->p2p_exchange = !(e && strcmp(e, "allgather") == 0) && c->world > 1;
     }
     if (c->p2p_exchange && c->local_form) {   // one process: plain peer access between every pair of devices
         for (RankCtx& a : c->ranks) {
@@ -775,11 +642,9 @@ frz_status comm_finish_setup(frz_comm* c) {
         if (c->world > 1) {
             FRZ_CUDA_TRY(cudaHostGetDevicePointer(&dp, c->tables.ptr, 0));
             r.table_dev = reinterpret_cast<uint32_t*>(dp);
-            const size_t entries = (size_t)c->world * kTableBins;
-            FRZ_CUDA_TRY(cudaMalloc(&r.d_pos0, entries * (sizeof(unsigned long long) + sizeof(uint32_t))));
-            r.d_gt = reinterpret_cast<uint32_t*>(r.d_pos0 + entries);
-            FRZ_CUDA_TRY(cudaMallocHost(&r.h_pos0, entries * (sizeof(unsigned long long) + sizeof(uint32_t))));
-            r.h_gt = reinterpret_cast<uint32_t*>(r.h_pos0 + entries);
+            const size_t table_bytes = (size_t)kTableBins * (sizeof(unsigned long long) + sizeof(uint32_t));
+            FRZ_CUDA_TRY(cudaMalloc(&r.d_pos0, table_bytes));
+            FRZ_CUDA_TRY(cudaMallocHost(&r.h_pos0, table_bytes));
         }
     }
     return FRZ_OK;
@@ -822,10 +687,10 @@ struct HostShard {
 };
 
 // Everything one GPU does for one match_list_parallel call.  `seq` is the step number shared by all ranks.
-// `want_slices`: the caller only needs the list in host memory (no device copy of the whole merged list): slice exchange allowed.
+// `host_only`: the caller only needs the list in host memory (no device copy of the whole merged list): P2P placement allowed.
 // Exactly one of `shard` (resident packed corpus) and `hs` (host buffers) is given.
 frz_status rank_step(frz_comm* c, RankCtx& r, frz_matcher* m, const frz_corpus* shard, const HostShard* hs, uint32_t index_offset, uint64_t seq,
-                     frz_match* out_host, uint64_t cap, bool want_host, bool want_slices, StepResult* res) {
+                     frz_match* out_host, uint64_t cap, bool want_host, bool host_only, StepResult* res) {
     FRZ_TRY(set_device(r.device));
     cudaStream_t main = nullptr;   // the device's legacy default stream: ordered with the caller's own default-stream work
     const int world = c->world;
@@ -868,13 +733,7 @@ frz_status rank_step(frz_comm* c, RankCtx& r, frz_matcher* m, const frz_corpus* 
     res->total = total;
     const bool collective = world > 1 || c->force_nccl;
     const FrzMatchDev* d_final = r.run;
-    uint64_t d_final_first = 0;   // merged position of d_final[0] (non-zero in the slice form)
-    bool placed = false;          // the P2P placement ran this step
-    bool direct_done = false;     // the direct form ran: this rank's matches went straight into the host buffer
-    // ---- host-out calls: SLICE EXCHANGE.  A rank copies only its slice [lo, hi) of the merged list to the host, and the
-    // elements of run q that land in that slice are ONE contiguous range of run q (a run's elements keep their order in the
-    // merged list).  With every rank's per-score table (published like the counts) each rank computes those ranges on the
-    // host and ONE grouped ncclSend/ncclRecv moves exactly them: 1/G of the all-gather's bytes and 1/G of its merge work.
+    uint64_t d_final_first = 0;   // merged position of d_final[0] (non-zero in the P2P form)
     const uint8_t sort_mode = frz_matcher_sort(m);
     const bool by_score = (sort_mode == FRZ_SORT_SCORE_THEN_INDEX_ASC || sort_mode == FRZ_SORT_SCORE_THEN_INDEX_DESC) &&
                           frz_matcher_num_patterns(m) > 0;
@@ -882,20 +741,18 @@ frz_status rank_step(frz_comm* c, RankCtx& r, frz_matcher* m, const frz_corpus* 
     int bins = 1;
     const uint32_t* d_table = nullptr;
     if (by_score) d_table = frz_matcher_last_sort_table(r.clone, &bins);
-    const bool slice_form = want_host && want_slices && world > 1 && r.nccl && c->slice_exchange && (!by_score || bins > 0) && total > 0 &&
-                            total <= 0xFFFFFFFFull;
-    if (slice_form) {
+    // ---- host-out calls: P2P PLACEMENT once the slice buffers are ready on every rank (collective, grow-only); otherwise the
+    // all-gather below, whose merged list every rank then copies its slice from
+    bool placed = false;          // the P2P placement runs this step
+    if (want_host && host_only && world > 1 && r.nccl && c->p2p_exchange && (!by_score || bins > 0) && total > 0 && total <= 0xFFFFFFFFull) {
         if (total > cap) {
             FRZ_CUDA_TRY(cudaStreamSynchronize(main));
             return frz_fail(FRZ_ERR_CAPACITY, "output capacity %llu < %llu matches", (unsigned long long)cap, (unsigned long long)total);
         }
         if (!out_host) return frz_fail(FRZ_ERR_INVALID_ARG, "null out");
-        // direct form: the caller's buffer mapped on every GPU?  Else the slice buffers of the P2P placement (collective,
-        // grow-only), else the NCCL slice exchange
-        FrzMatchDev* direct_out = nullptr;
-        FRZ_TRY(negotiate_direct(c, r, out_host, cap, &direct_out));
-        bool place_ready = direct_out != nullptr;
-        if (!direct_out) FRZ_TRY(ensure_place_buffers(c, r, total / (uint64_t)world + 2, &place_ready));
+        FRZ_TRY(ensure_place_buffers(c, r, total / (uint64_t)world + 2, &placed));
+    }
+    if (placed) {
         // 1. my table → shared block (after the local pipeline on the main stream), everybody's tables ← shared block
         volatile uint32_t* tab_host = c->tables_host + ((size_t)parity * world) * kTableBins;
         if (by_score) {
@@ -911,13 +768,10 @@ frz_status rank_step(frz_comm* c, RankCtx& r, frz_matcher* m, const frz_corpus* 
             FRZ_CUDA_TRY(cudaGetLastError());
             FRZ_TRY(wait_slots(c->ctrl_host + kCtrlTable + parity * kMaxWorld, world, seq, nullptr, "score table"));
         }
-        // 2. merged positions: pos0[q][s] = everything scoring higher than s in any run + the score-s blocks of the runs
-        //    that precede q in merge order; A[q][p] = how many elements of run q lie before slice boundary lo_p
-        uint64_t lo_p[kMaxWorld + 1];
-        for (int p2 = 0; p2 <= world; p2++) lo_p[p2] = total * (uint64_t)p2 / (uint64_t)world;
-      if (place_ready) {
-        // ---- P2P PLACEMENT: only MY run's rows of pos0 / gt are needed; k_place stores every element of my run at its merged
-        // position inside the owning rank's slice buffer (peer memory over NVLink) and ends when all peers have done the same
+        // 2. merged positions of MY run: pos0[s] = everything scoring higher than s in any run + the score-s blocks of the runs
+        //    that precede mine in merge order, gt[s] = how many of my run score higher than s.  k_place stores every element
+        //    of my run at its merged position inside the owning rank's slice buffer (peer memory over NVLink) and ends when
+        //    all peers have done the same
         auto gt_at = [&](int q, int sc) -> uint64_t { return by_score ? (uint64_t)tab_host[(size_t)q * kTableBins + sc] : 0ull; };
         uint64_t* hp = reinterpret_cast<uint64_t*>(r.h_pos0);
         uint32_t* hg = reinterpret_cast<uint32_t*>(hp + bins);
@@ -935,94 +789,15 @@ frz_status rank_step(frz_comm* c, RankCtx& r, frz_matcher* m, const frz_corpus* 
         PlaceMeta meta;
         memset(&meta, 0, sizeof meta);
         for (int q = 0; q < world; q++) meta.peer[q] = r.peer_raw[q];
-        for (int p2 = 0; p2 <= world; p2++) meta.lo[p2] = lo_p[p2];
+        for (int p = 0; p <= world; p++) meta.lo[p] = total * (uint64_t)p / (uint64_t)world;
         meta.total = total; meta.world = world; meta.rank = r.rank; meta.bins = bins; meta.parity = parity;
         const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((counts[r.rank] + 255) / 256, 148 * 4));
-        if (direct_out) {
-            k_place<true><<<grid, 256, 0, main>>>(r.run, counts[r.rank], meta, reinterpret_cast<const unsigned long long*>(r.d_pos0),
-                                                  reinterpret_cast<const uint32_t*>(r.d_pos0 + bins), seq, 0ull, nullptr, direct_out);
-            FRZ_CUDA_TRY(cudaGetLastError());
-            direct_done = true;   // my part of the list is already on its way to the host buffer: no slice copy
-        } else {
-            k_place<false><<<grid, 256, 0, main>>>(r.run, counts[r.rank], meta, reinterpret_cast<const unsigned long long*>(r.d_pos0),
-                                                   reinterpret_cast<const uint32_t*>(r.d_pos0 + bins), seq,
-                                                   (unsigned long long)(poll_timeout_s() * 1e9),
-                                                   reinterpret_cast<volatile unsigned long long*>(r.ctrl_dev + kCtrlPlaceErr + r.rank), nullptr);
-            FRZ_CUDA_TRY(cudaGetLastError());
-            placed = true;
-            d_final = reinterpret_cast<const FrzMatchDev*>(r.place_raw + kPlaceHeaderBytes);
-            d_final_first = lo_p[r.rank];
-        }
-      } else {
-        static thread_local std::vector<uint64_t> A;
-        A.assign((size_t)world * (world + 1), 0);
-        auto gt_of = [&](int q, int sc) -> uint64_t { return by_score ? (uint64_t)tab_host[(size_t)q * kTableBins + sc] : 0ull; };
-        for (int sc = bins - 1; sc >= 0; sc--) {
-            uint64_t higher = 0;
-            for (int q = 0; q < world; q++) higher += gt_of(q, sc);
-            uint64_t acc = higher;
-            for (int k = 0; k < world; k++) {
-                const int q = reversed ? world - 1 - k : k;
-                const uint64_t gtq = gt_of(q, sc);
-                const uint64_t ge = sc == 0 ? counts[q] : gt_of(q, sc - 1);
-                const uint64_t size = ge - gtq;
-                r.h_pos0[(size_t)q * bins + sc] = acc;
-                r.h_gt[(size_t)q * bins + sc] = (uint32_t)gtq;
-                if (size) {
-                    for (int p2 = 0; p2 <= world; p2++) {
-                        const uint64_t b = lo_p[p2];
-                        if (b > acc) A[(size_t)q * (world + 1) + p2] += std::min<uint64_t>(b - acc, size);
-                    }
-                }
-                acc += size;
-            }
-        }
-        // 3. ONE grouped exchange: to every rank p the part of my run it needs, from every run q the part I need
-        const uint64_t lo = lo_p[r.rank], hi = lo_p[r.rank + 1];
-        const uint64_t mine = hi - lo;
-        if (r.recv_cap < std::max<uint64_t>(mine, 1)) {
-            cudaFree(r.recv); r.recv = nullptr; r.recv_cap = 0;
-            const uint64_t want = mine + mine / 4 + 1024;
-            FRZ_CUDA_TRY(cudaMalloc(&r.recv, want * sizeof(FrzMatchDev)));
-            r.recv_cap = want;
-        }
-        if (r.merged_cap < std::max<uint64_t>(mine, 1)) {
-            cudaFree(r.merged); r.merged = nullptr; r.merged_cap = 0;
-            const uint64_t want = mine + mine / 4 + 1024;
-            FRZ_CUDA_TRY(cudaMalloc(&r.merged, want * sizeof(FrzMatchDev)));
-            r.merged_cap = want;
-        }
-        SliceMeta meta;
-        memset(&meta, 0, sizeof meta);
-        meta.lo = lo;
-        uint64_t off = 0, longest = 0;
-        for (int q = 0; q < world; q++) {
-            const uint64_t a = A[(size_t)q * (world + 1) + r.rank], b = A[(size_t)q * (world + 1) + r.rank + 1];
-            meta.off[q] = (uint32_t)off; meta.n[q] = (uint32_t)(b - a); meta.a[q] = (uint32_t)a;
-            off += b - a;
-            longest = std::max(longest, b - a);
-        }
-        if (off != mine) return frz_fail(FRZ_ERR_NCCL, "slice exchange: the ranks' score tables are inconsistent (%llu != %llu)",
-                                         (unsigned long long)off, (unsigned long long)mine);
-        FRZ_CUDA_TRY(cudaMemcpyAsync(r.d_pos0, r.h_pos0, (size_t)world * kTableBins * (sizeof(unsigned long long) + sizeof(uint32_t)),
-                                     cudaMemcpyHostToDevice, main));   // pos0 and gt in one copy (fixed layout, <= 96 KB)
-        FRZ_NCCL_TRY(nccl_api().GroupStart());
-        for (int p2 = 0; p2 < world; p2++) {
-            const uint64_t a = A[(size_t)r.rank * (world + 1) + p2], b = A[(size_t)r.rank * (world + 1) + p2 + 1];
-            if (b > a) FRZ_NCCL_TRY(nccl_api().Send(r.run + a, (size_t)(b - a), ncclUint64, p2, r.nccl, main));
-        }
-        for (int q = 0; q < world; q++)
-            if (meta.n[q]) FRZ_NCCL_TRY(nccl_api().Recv(r.recv + meta.off[q], (size_t)meta.n[q], ncclUint64, q, r.nccl, main));
-        FRZ_NCCL_TRY(nccl_api().GroupEnd());
-        // 4. my slice of the k-way merge
-        if (mine) {
-            const dim3 grid((unsigned)std::max<uint64_t>(1, std::min<uint64_t>((longest + 255) / 256, 148 * 4 / world + 1)), (unsigned)world);
-            k_slice_scatter<<<grid, 256, 0, main>>>(r.recv, meta, r.d_gt, r.d_pos0, bins, r.merged);
-            FRZ_CUDA_TRY(cudaGetLastError());
-        }
-        d_final = r.merged;
-        d_final_first = lo;
-      }
+        k_place<<<grid, 256, 0, main>>>(r.run, counts[r.rank], meta, reinterpret_cast<const unsigned long long*>(r.d_pos0),
+                                        reinterpret_cast<const uint32_t*>(r.d_pos0 + bins), seq, (unsigned long long)(poll_timeout_s() * 1e9),
+                                        reinterpret_cast<volatile unsigned long long*>(r.ctrl_dev + kCtrlPlaceErr + r.rank));
+        FRZ_CUDA_TRY(cudaGetLastError());
+        d_final = reinterpret_cast<const FrzMatchDev*>(r.place_raw + kPlaceHeaderBytes);
+        d_final_first = meta.lo[r.rank];
     } else if (collective) {
         if (r.run_cap < stride) {
             // another rank's run is longer than this rank's whole shard (ceil partitioning leaves the last shard short, or
@@ -1058,7 +833,7 @@ frz_status rank_step(frz_comm* c, RankCtx& r, frz_matcher* m, const frz_corpus* 
         FRZ_TRY(frz_merge_runs_ex(r.merge, r.gathered, stride, counts, world, frz_matcher_sort(m), frz_matcher_score_bound(m), r.merged, main));
         d_final = r.merged;
     }
-    res->d_merged = slice_form ? nullptr : d_final;
+    res->d_merged = placed ? nullptr : d_final;
     FRZ_CUDA_TRY(cudaEventRecord(r.ev[2], main));
     if (want_host) {
         if (total > cap) {   // every rank sees the same counts, so every rank takes this exit: no collective is left unbalanced
@@ -1068,7 +843,7 @@ frz_status rank_step(frz_comm* c, RankCtx& r, frz_matcher* m, const frz_corpus* 
         if (total && !out_host) return frz_fail(FRZ_ERR_INVALID_ARG, "null out");
         // this rank's slice of the merged list → host (all ranks hold the whole list: the copy uses every PCIe link)
         const uint64_t lo = total * (uint64_t)r.rank / (uint64_t)world, hi = total * (uint64_t)(r.rank + 1) / (uint64_t)world;
-        if (hi > lo && !direct_done)
+        if (hi > lo)
             FRZ_CUDA_TRY(cudaMemcpyAsync(out_host + lo, d_final + (lo - d_final_first), (hi - lo) * sizeof(FrzMatchDev), cudaMemcpyDeviceToHost, main));
     }
     FRZ_CUDA_TRY(cudaEventRecord(r.ev[3], main));
@@ -1182,7 +957,7 @@ extern "C" int frz_comm_rank(const frz_comm* c) { return c ? c->rank : -1; }
 extern "C" int frz_comm_device(const frz_comm* c, int i) { return (c && i >= 0 && i < (int)c->ranks.size()) ? c->ranks[i].device : -1; }
 
 extern "C" int frz_comm_exchange_mode(const frz_comm* c) {
-    return !c ? -1 : (c->direct_exchange && c->world > 1) ? 3 : (c->p2p_exchange && c->world > 1) ? 2 : c->slice_exchange ? 1 : 0;
+    return !c ? -1 : c->p2p_exchange ? 2 : 0;
 }
 
 extern "C" frz_status frz_comm_host_alloc(frz_comm* c, uint64_t bytes, void** out) {
@@ -1198,7 +973,7 @@ extern "C" frz_status frz_comm_host_free(frz_comm* c, void* p) {
     if (!c || !p) return FRZ_OK;
     for (size_t i = 0; i < c->blocks.size(); i++)
         if (c->blocks[i].ptr == p) {
-            for (RankCtx& r : c->ranks) { cudaSetDevice(r.device); cudaDeviceSynchronize(); r.direct_for = nullptr; r.direct_dev = nullptr; }
+            for (RankCtx& r : c->ranks) { cudaSetDevice(r.device); cudaDeviceSynchronize(); }
             host_block_release(c->blocks[i]);
             c->blocks.erase(c->blocks.begin() + (long)i);
             return FRZ_OK;

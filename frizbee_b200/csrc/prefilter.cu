@@ -507,8 +507,9 @@ struct __align__(16) CandRec {
 // ---- TMA staging (cp.async.bulk, 1-D) of the phase-A arrays ---------------------------------------------------------
 // The metadata, signature and group-descriptor arrays are contiguous, so a warp's next 128-slot chunk is three bulk
 // copies (512 + 1024 + 64 bytes) that complete on the warp's OWN mbarrier: warp-autonomous, no block barrier, and the
-// bytes in flight hold no registers (the register-prefetch form, kept below as the A/B partner, pays 14 registers per
-// chunk in flight and ptxas sinks such loads towards their use).  Three stages per warp.
+// bytes in flight hold no registers (a register-prefetch form pays 14 registers per chunk in flight and ptxas sinks such
+// loads towards their use: it measured 0.1596 against 0.1568 ms for the stage, profiles/r02_experiments.md).  Three stages
+// per warp.
 constexpr int kScanStages = 3;
 struct __align__(16) ScanStage {
     uint32_t meta[128];
@@ -541,10 +542,9 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
         : "memory");
 }
 
-template <bool TMA>
-__global__ void __launch_bounds__(kScanThreads, TMA ? 6 : 10) k_sig_scan(const FrzCorpusView cv, int use_sig, uint32_t need1, uint32_t need2,
-                                                                         int sig_k, int min_len, CandRec* __restrict__ cand,
-                                                                         unsigned long long cand_cap, FrzCounters* __restrict__ ctr) {
+__global__ void __launch_bounds__(kScanThreads, 6) k_sig_scan(const FrzCorpusView cv, int use_sig, uint32_t need1, uint32_t need2,
+                                                               int sig_k, int min_len, CandRec* __restrict__ cand,
+                                                               unsigned long long cand_cap, FrzCounters* __restrict__ ctr) {
     extern __shared__ __align__(16) unsigned char scan_smem[];
     const uint32_t lane = frz_lane(), warp = threadIdx.x >> 5;
     CandRec* ring = reinterpret_cast<CandRec*>(scan_smem) + (size_t)warp * kScanRing;
@@ -596,7 +596,7 @@ __global__ void __launch_bounds__(kScanThreads, TMA ? 6 : 10) k_sig_scan(const F
         while (count >= 32) flush_request(32);
         __syncwarp();
     };
-    if constexpr (TMA) {
+    {   // the chunk pipeline: three TMA stages per warp, each completing on its own mbarrier
         ScanStage* stages = reinterpret_cast<ScanStage*>(scan_smem + sizeof(CandRec) * kScanRing * kScanWarps) + warp * kScanStages;
         uint64_t* bars = reinterpret_cast<uint64_t*>(scan_smem + (sizeof(CandRec) * kScanRing + sizeof(ScanStage) * kScanStages) * kScanWarps) +
                          warp * kScanStages;
@@ -638,49 +638,6 @@ __global__ void __launch_bounds__(kScanThreads, TMA ? 6 : 10) k_sig_scan(const F
             cur += n_warps;
             if (++st == kScanStages) { st = 0; parity ^= 1; }
         }
-    } else {
-        // register prefetch: two chunk buffers ping-pong, the other buffer's loads are in flight while one is tested
-        struct Chunk {
-            uint4 meta;
-            uint4 sig0, sig1;
-            unsigned long long abs_off;   // lanes 0-3: first unit of the chunk's group `lane`
-            uint32_t gunits;              // lanes 0-3: units per slot of that group
-            uint32_t idx;
-        };
-        uint32_t next = blockIdx.x * kScanWarps + warp;
-        auto load_chunk = [&](Chunk& c) {
-            c.idx = next < total_chunks ? next : 0xFFFFFFFFu;
-            c.meta = make_uint4(FRZ_INVALID_SLOT, FRZ_INVALID_SLOT, FRZ_INVALID_SLOT, FRZ_INVALID_SLOT);
-            c.sig0 = c.sig1 = make_uint4(0u, 0u, 0u, 0u);
-            c.abs_off = 0;
-            c.gunits = 0;
-            if (next < total_chunks) {
-                const uint64_t slot0 = (uint64_t)next * 128 + lane * 4;
-                c.meta = __ldg(reinterpret_cast<const uint4*>(cv.slot_meta + slot0));
-                if (use_sig) {
-                    const uint4* sp = reinterpret_cast<const uint4*>(cv.slot_sig + slot0);
-                    c.sig0 = __ldg(sp);
-                    c.sig1 = __ldg(sp + 1);
-                }
-                if (lane < 4) {   // four contiguous 16-byte descriptors, L2-resident
-                    const FrzGroupDesc gd = cv.groups[next * 4 + lane];
-                    c.abs_off = gd.abs_off;
-                    c.gunits = gd.gunits;
-                }
-            }
-            next += n_warps;
-        };
-        Chunk ca, cb;
-        load_chunk(ca);
-        load_chunk(cb);
-        for (;;) {
-            if (ca.idx == 0xFFFFFFFFu) break;
-            process(ca.idx, ca.meta, ca.sig0, ca.sig1, __shfl_sync(0xffffffffu, ca.abs_off, lane >> 3), __shfl_sync(0xffffffffu, ca.gunits, lane >> 3));
-            load_chunk(ca);
-            if (cb.idx == 0xFFFFFFFFu) break;
-            process(cb.idx, cb.meta, cb.sig0, cb.sig1, __shfl_sync(0xffffffffu, cb.abs_off, lane >> 3), __shfl_sync(0xffffffffu, cb.gunits, lane >> 3));
-            load_chunk(cb);
-        }
     }
     flush_commit();
     if (count) { flush_request(count); flush_commit(); }
@@ -708,8 +665,7 @@ template <int MODE>
 __global__ void __launch_bounds__(kWinThreads, 4) k_window(const FrzCorpusView cv, const __grid_constant__ FrzPatternDev pat,
                                                            const CandRec* __restrict__ cand, unsigned long long cand_cap,
                                                            const FrzSurvLists lists, unsigned long long surv_cap,
-                                                           uint32_t* __restrict__ surv_bitmap, FrzCounters* __restrict__ ctr,
-                                                           uint32_t flags) {
+                                                           uint32_t* __restrict__ surv_bitmap, FrzCounters* __restrict__ ctr) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const uint32_t lane = frz_lane(), warp = threadIdx.x >> 5;
     WinSmem& sm = reinterpret_cast<WinSmem*>(smem_raw)[warp];
@@ -719,7 +675,7 @@ __global__ void __launch_bounds__(kWinThreads, 4) k_window(const FrzCorpusView c
     const unsigned long long n_cand = min(ctr->cand_count, cand_cap);
     const uint32_t n_items = (uint32_t)((n_cand + 31) >> 5);
     const bool staged = cv.max_gunits <= 4;   // every haystack fits the four staged units
-    const bool single = (MODE == FRZ_T_0 || MODE == FRZ_T_1) && (flags & 1u) && single_chunk_ok(pat, cv.max_gunits);
+    const bool single = (MODE == FRZ_T_0 || MODE == FRZ_T_1) && single_chunk_ok(pat, cv.max_gunits);
 
     // Work items are strided statically over the warps of the grid (their cost is uniform), so the item sequence of a warp
     // is known ahead: item k's units AND item k+1's records were requested with cp.async one iteration earlier (records
@@ -977,28 +933,19 @@ frz_status frz_launch_sig_scan(const FrzCorpusView& cv, const FrzPatternDev& pat
     if (sms <= 0) sms = 148;
     CandRec* cand = reinterpret_cast<CandRec*>(ws.cand_list);
     {   // persistent warps, as many blocks as fit
-        static int tma_knob = -1;   // A/B knob: FRZ_PF_TMA=0 selects the register-prefetch form of the phase-A loads
-        if (tma_knob < 0) { const char* e = getenv("FRZ_PF_TMA"); tma_knob = e ? atoi(e) : 1; }
         const uint32_t total_chunks = cv.n_tiles * (FRZ_TILE / 128);
         const int use_sig = pat.typo_mode != FRZ_T_NONE && pat.sig_on;
-        const size_t ring_bytes = sizeof(CandRec) * kScanRing * kScanWarps;
-        const size_t smem_tma = ring_bytes + (sizeof(ScanStage) * kScanStages + sizeof(uint64_t) * kScanStages) * kScanWarps;
-#define FRZ_SCAN_LAUNCH(TMA, SMEM)                                                                                       \
-        do {                                                                                                             \
-            static int bps_dev[64] = {};                                                                                 \
-            int& bps = bps_dev[frz_current_device() & 63];                                                               \
-            if (!bps) {                                                                                                  \
-                FRZ_CUDA_TRY(cudaFuncSetAttribute(k_sig_scan<TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SMEM))); \
-                FRZ_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_sig_scan<TMA>, kScanThreads, (SMEM))); \
-                if (bps < 1) bps = 1;                                                                                    \
-            }                                                                                                            \
-            const uint32_t grid = std::max<uint32_t>(1, std::min<uint32_t>((uint32_t)(sms * bps), (total_chunks + kScanWarps - 1) / kScanWarps)); \
-            k_sig_scan<TMA><<<grid, kScanThreads, (SMEM), stream>>>(cv, use_sig, pat.sig_need1, pat.sig_need2, pat.sig_k,  \
-                                                                   pat.min_hay_len, cand, ws.cand_cap, ws.counters);     \
-        } while (0)
-        if (tma_knob) FRZ_SCAN_LAUNCH(true, smem_tma);
-        else FRZ_SCAN_LAUNCH(false, ring_bytes);
-#undef FRZ_SCAN_LAUNCH
+        const size_t smem = (sizeof(CandRec) * kScanRing + sizeof(ScanStage) * kScanStages + sizeof(uint64_t) * kScanStages) * kScanWarps;
+        static int bps_dev[64] = {};
+        int& bps = bps_dev[frz_current_device() & 63];
+        if (!bps) {
+            FRZ_CUDA_TRY(cudaFuncSetAttribute(k_sig_scan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            FRZ_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_sig_scan, kScanThreads, smem));
+            if (bps < 1) bps = 1;
+        }
+        const uint32_t grid = std::max<uint32_t>(1, std::min<uint32_t>((uint32_t)(sms * bps), (total_chunks + kScanWarps - 1) / kScanWarps));
+        k_sig_scan<<<grid, kScanThreads, smem, stream>>>(cv, use_sig, pat.sig_need1, pat.sig_need2, pat.sig_k, pat.min_hay_len, cand,
+                                                         ws.cand_cap, ws.counters);
     }
     FRZ_CUDA_TRY(cudaGetLastError());
     if (st) st->launches++;
@@ -1015,9 +962,6 @@ frz_status frz_launch_prefilter(const FrzCorpusView& cv, const FrzPatternDev& pa
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (sms <= 0) sms = 148;
     FRZ_CUDA_TRY(cudaMemsetAsync(ws.surv_bitmap, 0, (size_t)cv.n_tiles * 32 * sizeof(uint32_t), stream));
-    static int single_knob = -1;   // A/B knob: FRZ_PF_SINGLE=0 keeps the general (multi-chunk) mask forms
-    if (single_knob < 0) { const char* e = getenv("FRZ_PF_SINGLE"); single_knob = e ? atoi(e) : 1; }
-    const uint32_t pf_flags = single_knob ? 1u : 0u;
     CandRec* cand = reinterpret_cast<CandRec*>(ws.cand_list);
     FRZ_TRY(frz_launch_sig_scan(cv, pat, ws, stream, st));   // 1a
     const size_t smem = sizeof(WinSmem) * kWinWarps;
@@ -1028,17 +972,14 @@ frz_status frz_launch_prefilter(const FrzCorpusView& cv, const FrzPatternDev& pa
         if (!bps) {                                                                                                      \
             FRZ_CUDA_TRY(cudaFuncSetAttribute(k_window<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));  \
             FRZ_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_window<MODE>, kWinThreads, smem));        \
-            static int knob = -1;   /* experiment knob: FRZ_PF_BLOCKS caps the resident blocks per SM */                 \
-            if (knob < 0) { const char* e = getenv("FRZ_PF_BLOCKS"); knob = e ? atoi(e) : 0; }                           \
             /* measured on B200, slot-major layout (profiles/r02j_variants.txt): 5 / 4 / 3 resident blocks per SM give */ \
             /* 0.1302 / 0.1328 / 0.1429 ms for the stage (with the interleaved layout 4 beat 5: each candidate touched */  \
             /* four lines and more warps thrashed L1, profiles/r02f_variants.txt) */                                      \
-            if (knob > 0) bps = std::min(bps, knob);                                                                     \
-            else if (bps > 5) bps = 5;                                                                                   \
+            if (bps > 5) bps = 5;                                                                                        \
             if (bps < 1) bps = 1;                                                                                        \
         }                                                                                                                \
         k_window<MODE><<<sms * bps, kWinThreads, smem, stream>>>(cv, pat, cand, ws.cand_cap, ws.lists(), ws.survivor_cap, \
-                                                                 ws.surv_bitmap, ws.counters, pf_flags);                 \
+                                                                 ws.surv_bitmap, ws.counters);                           \
     } while (0)
     switch (pat.typo_mode) {
         case FRZ_T_0: FRZ_PF_LAUNCH(FRZ_T_0); break;

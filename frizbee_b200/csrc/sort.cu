@@ -212,6 +212,6 @@ frz_status frz_sort_hist_alloc(uint32_t** out) {
 
 // digit_base[d] of the LAST pass run on this workspace = number of elements whose digit is greater than d.  After a
 // single-pass sort (score bound < 1024) that is, per score s, how many matches of the run score higher than s — the table
-// the multi-GPU slice exchange needs (parallel.cu) — so nobody has to binary-search the sorted run for it.
+// the multi-GPU P2P placement needs (parallel.cu) — so nobody has to binary-search the sorted run for it.
 const uint32_t* frz_sort_digit_base(const FrzWorkspace& ws) { return ws.sort_hist ? ws.sort_hist + (size_t)kMaxBins * kV + kMaxBins : nullptr; }
 int frz_sort_single_pass_bins(uint32_t score_bound) { return score_bound < 256 ? 256 : score_bound < 512 ? 512 : score_bound < 1024 ? 1024 : 0; }

@@ -116,7 +116,7 @@ class Comm:
         _check(plib().frz_comm_barrier(self._h))
 
     def exchange_mode(self) -> int:
-        """3 = direct placement into the mapped host buffer, 2 = P2P placement, 1 = NCCL slice exchange, 0 = all-gather."""
+        """How host-out calls move the matches: 2 = P2P placement, 0 = all-gather."""
         return int(plib().frz_comm_exchange_mode(self._h))
 
     def p2p_active(self) -> bool:
@@ -151,7 +151,7 @@ class Comm:
         """Multi-process form (frz_match_list_parallel_rank), collective.  `out`: the SHARED host array from
         host_alloc_matches (every rank passes its mapping) or None for a device-only result.  `want_device` (default: only
         when `out` is None) also asks for this rank's device copy of the WHOLE merged list — that forces the all-gather form;
-        host-only calls use the slice exchange.  Returns (total matches, device pointer of the merged list or 0)."""
+        host-only calls use the P2P placement when peer memory is mapped.  Returns (total matches, device pointer of the merged list or 0)."""
         if want_device is None:
             want_device = out is None
         n = C.c_uint64()

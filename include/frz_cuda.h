@@ -286,14 +286,11 @@ FRZ_API frz_status frz_match_list_parallel_rank(frz_matcher* m, const frz_corpus
 FRZ_API frz_status frz_match_list_parallel_rank_host(frz_matcher* m, const uint8_t* bytes, const void* offsets, int offset_width,
                                              uint64_t n, uint32_t index_offset, frz_comm* c, frz_match* out, uint64_t cap,
                                              uint64_t* n_out);
-/* How host-out calls move the matches on this communicator: 3 = direct placement (every GPU stores its matches at their
- * merged positions straight into the caller's pinned + mapped host buffer — frz_comm_host_alloc memory — over its own
- * PCIe link; a buffer that is not mapped on every GPU uses form 2 for that call), 2 = P2P placement (into the peers' slice
- * buffers over NVLink — peer access in the local form, cudaIpc in the multi-process form — then every GPU copies its slice
- * out), 1 = NCCL slice exchange (grouped ncclSend/ncclRecv), 0 = ncclAllGather of whole runs + merge.  Chosen at creation
- * (FRZ_PARALLEL_EXCHANGE=direct|p2p|slices|allgather, default p2p — measured faster than direct on B200, where the copy
- * engine moves a slice at ~52 GB/s and SM-issued stores to host memory reach ~30 GB/s); 2 is downgraded to 1 by the first
- * call when peer memory cannot be mapped.  Device-out calls always use the all-gather. */
+/* How host-out calls move the matches on this communicator: 2 = P2P placement (every GPU stores its matches at their
+ * merged positions in the peers' slice buffers over NVLink — peer access in the local form, cudaIpc in the multi-process
+ * form — then every GPU copies its slice out), 0 = ncclAllGather of whole runs + merge.  Chosen at creation (default 2 on
+ * more than one GPU; FRZ_PARALLEL_EXCHANGE=allgather selects 0); 2 is downgraded to 0 by the first call when peer memory
+ * cannot be mapped.  1 and 3 are no longer returned.  Device-out calls always use the all-gather. */
 FRZ_API int frz_comm_exchange_mode(const frz_comm* c);
 
 /* Device timings (ms) of the last parallel call on local rank `local_index`: [0] local pipeline (prefilter, scoring,

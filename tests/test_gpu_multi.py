@@ -154,12 +154,11 @@ def test_c_client_on_the_gpu(tmp_path):
     assert f"match_list_parallel over {n} GPU(s)" in r.stdout and "parallel == sequential: yes" in r.stdout
 
 
-@pytest.mark.parametrize("exchange", ["direct", "p2p", "slices", "allgather"])
+@pytest.mark.parametrize("exchange", ["p2p", "allgather"])
 def test_local_form_two_gpus(exchange, monkeypatch):
-    """Single process, two GPUs (frz_comm_create_local: ncclCommInitAll + one worker thread per GPU), with all four forms of
-    the exchange step: direct placement into the mapped host buffer (k_place<DIRECT>), P2P placement (k_place: every GPU stores its matches at their merged positions in the peers' slice
-    buffers over NVLink), the slice exchange (grouped ncclSend/ncclRecv of exactly what each rank copies out) and the
-    all-gather of whole runs."""
+    """Single process, two GPUs (frz_comm_create_local: ncclCommInitAll + one worker thread per GPU), with both forms of
+    the exchange step: P2P placement (k_place: every GPU stores its matches at their merged positions in the peers' slice
+    buffers over NVLink) and the all-gather of whole runs."""
     if _gpus() < 2:
         pytest.skip("needs >= 2 GPUs")
     import frizbee_b200 as F
@@ -189,9 +188,9 @@ def test_local_form_two_gpus(exchange, monkeypatch):
     whole.close(); comm.close()
 
 
-@pytest.mark.parametrize("exchange", ["direct", "p2p", "slices", "allgather"])
+@pytest.mark.parametrize("exchange", ["p2p", "allgather"])
 def test_match_list_parallel_two_gpus_torchrun(exchange):
-    """One rank per GPU under torchrun (the bench's launch mode): tests/_multi_gpu_worker.py, with all four forms of the
+    """One rank per GPU under torchrun (the bench's launch mode): tests/_multi_gpu_worker.py, with both forms of the
     exchange step for the host-out calls (device-only calls always all-gather; p2p maps the peers' slice buffers with cudaIpc)."""
     if _gpus() < 2:
         pytest.skip("needs >= 2 GPUs")
